@@ -2,7 +2,7 @@
 """bench.py -- frames/sec of the attention-lvcsr hot path (encoder + teacher-forced
 attention decoder) at the BASELINE.json metric configuration.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one pass of the hot path over one synthetic batch per GPU:
@@ -176,6 +176,17 @@ def cpu_reference_run(steps, warmup, sample_B=64):
         value=fps, unit="frames/s", cores=cores, kind="port",
         sample="%d utterances x %d frames x %d fbank, %d decoder steps, float32 numpy+BLAS restatement of the "
                "Theano CPU path (Theano itself cannot run: SURVEY.md 8c)" % (sample_B, W["T"], W["F"], W["L"]))
+
+
+def dump_outputs(arrays, path, limit=64 * 10 ** 6):
+    """Write each float32 array (utterances on axis 1) as path/<name>.npy, at most `limit` bytes in all: past
+    that, every array keeps the same leading utterances, as many as fit, so that runs stay comparable."""
+    B = next(iter(arrays.values())).shape[1]
+    per_utt = sum(a.nbytes for a in arrays.values()) / B
+    keep = min(B, int((limit - 1024 * len(arrays)) // per_utt))       # 1 KiB per .npy header, generously
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a[:, :keep]))
 
 
 TRAIN_WORKLOAD = dict(B=64, T=1500, F=40, L=190, V=32)       # BASELINE.json configs[3]
@@ -458,7 +469,15 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="metric mode: skip the training-step block")
     ap.add_argument("--batch", type=int, default=WORKLOAD["B"],
                     help="diagnostic only: utterances per GPU (the metric is quoted on the default)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="metric mode: write what the last timed step returned (costs [L,B], attended [T',B,E], "
+                         "attended_mask [T',B]) for rank 0's shard as DIR/<name>.npy in float32, at most 64 MB "
+                         "(the default batch takes 33 MB; a larger --batch keeps its first utterances)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.mode != "metric" or args.impl != "ours"):
+        ap.error("--dump-outputs is only supported with --mode metric --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -474,12 +493,11 @@ def main():
     if args.impl == "reference":
         if rank != 0:
             return 0
-        steps = max(1, min(args.steps, 2))
-        fps, ms, cb = cpu_reference_run(steps, 0)
+        fps, ms, cb = cpu_reference_run(args.steps, 0)
         config["reference_sample_B"] = 64
         print(json.dumps({
             "impl": "reference", "metric": METRIC, "value": fps, "unit": "frames/s", "n_gpus": args.gpus,
-            "steps": steps, "warmup": 0, "ms_per_step": ms, "higher_is_better": True,
+            "steps": args.steps, "warmup": 0, "ms_per_step": ms, "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic", "config": config,
             "cpu_baseline": cb,
             "e2e": {"value": fps, "unit": "frames/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}}))
@@ -513,7 +531,7 @@ def main():
 
     def step_device():
         att, attm = rec.encode(xd, md)
-        return rec.cost_matrix(yd, ymd, att, attm)
+        return {"costs": rec.cost_matrix(yd, ymd, att, attm), "attended": att, "attended_mask": attm}
 
     def step_host():
         return rec.cost(xh.numpy(), mh.numpy(), yh.numpy(), ymh.numpy())
@@ -526,17 +544,20 @@ def main():
         torch.cuda.synchronize(dev)
 
     def timed(fn, steps):
+        """Device time of `steps` calls and what the last call returned."""
         total_ms = 0.0
-        for _ in range(steps):
+        for i in range(steps):
             flush.fill_(1)                       # evict L2 between timed iterations
             torch.cuda.synchronize(dev)
             a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
-            fn()
+            out = fn()
             b.record()
             torch.cuda.synchronize(dev)
             total_ms += a.elapsed_time(b)
-        return total_ms
+            if i < steps - 1:
+                out = None                       # free it so that the next step reuses its memory
+        return total_ms, out
 
     dist_mod = None
     if world > 1:
@@ -546,11 +567,11 @@ def main():
         sampler = ClockSampler(local_rank)
         sampler.start()
         if args.mode == "search":
-            sr = search_bench(pkg, torch, dev, rank, world, max(1, min(args.steps, 3)), 1, dist_mod, barrier,
+            sr = search_bench(pkg, torch, dev, rank, world, args.steps, 1, dist_mod, barrier,
                               cpu_baseline=not args.no_cpu_baseline)
             main_case = sr["config3_beam10"]
             line = {"metric": SEARCH_METRIC, "value": main_case["utterances_per_s"], "unit": "utterances/s", "n_gpus": world,
-                    "steps": max(1, min(args.steps, 3)), "warmup": 1, "ms_per_step": main_case["ms_per_batch"],
+                    "steps": args.steps, "warmup": 1, "ms_per_step": main_case["ms_per_batch"],
                     "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
                     "config": {"workload": "configs[2]: 32 utterances x <=800 frames per GPU, beam_size 10; configs[0] in `search`",
                                "parallelism": "dp%d (utterances sharded, no cross-device traffic)" % world},
@@ -593,7 +614,10 @@ def main():
     sampler.start()
     lib.lvsr_launch_count(1)
     barrier()
-    ms_dev = timed(step_device, args.steps)
+    ms_dev, last = timed(step_device, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs({k: v.float().cpu().numpy() for k, v in last.items()}, args.dump_outputs)
+    del last
     barrier()
     launches = int(lib.lvsr_launch_count(1))
     ms_dev = max_over_ranks(ms_dev, world, dev, dist_mod)
@@ -624,7 +648,7 @@ def main():
     train_block = None
     if not args.no_train and args.batch == WORKLOAD["B"]:
         try:
-            train_block = train_bench(pkg, torch, dev, rank, world, max(2, min(args.steps, 5)), 2, dist_mod, flush, barrier)
+            train_block = train_bench(pkg, torch, dev, rank, world, args.steps, 2, dist_mod, flush, barrier)
         except Exception as e:          # the headline must survive a failure of the secondary measurement
             train_block = {"error": "%s: %s" % (type(e).__name__, e)}
 

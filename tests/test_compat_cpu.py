@@ -3,8 +3,6 @@ import os
 import subprocess
 import sys
 
-import pytest
-
 from compat_helpers import COMPAT, ROOT, write_experiment
 
 
@@ -53,15 +51,34 @@ def test_dataset_batches_are_time_major_padded_and_masked(tmp_path):
     assert n == 10
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/bin/run.py"), reason="the reference tree is not on this machine")
+# Replays a call recorded from the reference's bin/run.py (tests/golden/make_run_py_golden.py): its imports, then
+# Configuration(...) and lvsr.main.<func>(config, **kwargs) with exactly the arguments run.py passed.
+RUN_PY_REPLAY = r"""
+import importlib, json, logging, sys
+call = json.loads(open(sys.argv[1]).read().replace("<tmp>", sys.argv[2]))
+for module, name in call["imports"]:
+    if name:
+        getattr(importlib.import_module(module), name)
+logging.basicConfig(level=call["logging_level"], format="%(asctime)s: %(name)s: %(levelname)s: %(message)s")
+from lvsr.config import Configuration
+import lvsr.main
+path, schema, changes = call["configuration_args"]
+config = Configuration(path, schema, [tuple(c) for c in changes])
+config["cmd_args"] = call["cmd_args"]
+getattr(lvsr.main, call["func"])(config, **call["kwargs"])
+"""
+
+
 def test_reference_run_py_runs_unchanged_up_to_the_device(tmp_path):
-    """`python <reference>/bin/run.py search ...` with PYTHONPATH=compat: argument parsing, Configuration and
-    lvsr.main.search are reached with the reference's UNMODIFIED entry script; without a GPU the first device call
-    fails loudly (no CPU fallback)."""
-    exp = write_experiment(tmp_path)
+    """The call the reference's UNMODIFIED bin/run.py makes for `run.py search <tmp>/missing.tar <tmp>/base.yaml
+    monitoring.search.beam_size 2` with PYTHONPATH=compat (recorded in tests/golden/run_py_search_call.json):
+    its imports resolve, Configuration and lvsr.main.search accept its arguments; without a GPU the first device
+    call fails loudly (no CPU fallback)."""
+    write_experiment(tmp_path)
     env = dict(os.environ, PYTHONPATH=COMPAT, CUDA_VISIBLE_DEVICES="")
-    r = subprocess.run([sys.executable, "/root/reference/bin/run.py", "search", os.path.join(str(tmp_path), "missing.tar"),
-                        exp["base"], "monitoring.search.beam_size", "2"], env=env, capture_output=True, text=True, timeout=300)
+    call = os.path.join(ROOT, "tests", "golden", "run_py_search_call.json")
+    r = subprocess.run([sys.executable, "-c", RUN_PY_REPLAY, call, str(tmp_path)], env=env, capture_output=True,
+                       text=True, timeout=300)
     out = r.stdout + r.stderr
     assert "Recognizer initialization started" in out, out[-2000:]
     assert r.returncode != 0 and ("CUDA" in out or "cuda" in out), out[-2000:]

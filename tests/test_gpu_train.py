@@ -153,7 +153,7 @@ def test_two_gpu_step_equals_single_gpu_step_on_the_concatenated_batch():
     """SURVEY.md 8e: batch sharded over ranks + ONE NCCL all-reduce of the flat gradient buffer."""
     torch = _torch()
     if torch.cuda.device_count() < 2:
-        pytest.skip("needs two GPUs (gpurun --gpus 2)")
+        pytest.skip("needs two GPUs")
     import os
     import subprocess
     import sys
