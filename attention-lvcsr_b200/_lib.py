@@ -71,6 +71,7 @@ SIGNATURES = {
     "lvsr_model_flat_params": (C.c_void_p, [_P]),
     "lvsr_model_finalize": (C.c_int, [_P]),
     "lvsr_model_status": (C.c_int, [_P, C.POINTER(C.c_int32), C.POINTER(C.c_int64)]),
+    "lvsr_dec_scan_plan": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "lvsr_encoded_length": (C.c_int, [_P, _I]),
     "lvsr_encoded_dim": (C.c_int, [_P]),
     "lvsr_encoder_forward": (C.c_int, [_P, _P, _P, _I, _I, _P, _P, _P]),

@@ -80,6 +80,10 @@ struct AttRowIO {
   float* rowpos_out = nullptr;
   int rowpos_mode = 0;
   unsigned long long* trace = nullptr;   // optional [8] globaltimer stamps (debug)
+  // P of this CTA's positions is resident in tensor memory (att_stage_p_tmem): the energies read it from
+  // there instead of L2.  p_taddr = this thread's TMEM address of tile 0 (att_p_taddr).
+  int p_tmem = 0;
+  uint32_t p_taddr = 0;
 };
 
 __device__ __forceinline__ unsigned long long att_global_ns() {
@@ -160,8 +164,95 @@ __device__ __forceinline__ void mma_bf16_16816(float (&d)[4], const uint32_t (&a
       : "r"(a[0]), "r"(a[1]), "r"(a[2]), "r"(a[3]), "r"(b0), "r"(b1));
 }
 
+// ---- P resident in tensor memory ---------------------------------------------------------
+// When a persistent caller's window is the whole utterance on every step, each CTA reads the same P
+// slice on every step.  It can instead keep that slice in its 512 TMEM columns: thread-private, in
+// exactly the order of the mma.sync accumulator fragments the energy loop initialises from P.  Warp w
+// may address TMEM lanes 32*(w%4)..+31 only, so the four warps of a lane quarter take 128 columns
+// each; a thread's tile k holds its 4*NTW accumulator values at columns [k*4*NTW, +4*NTW):
+//   column j*4 + {0, 1, 2, 3} = P[row g][n0 + 2tig], P[row g][n0 + 2tig + 1], P[row g+8][...], P[row g+8][... + 1]
+// of the 16-position tile (n0 = first column of the warp's j-th 8-column tile).  Fits when
+// ceil(tc_cap / 16) * 4 * NTW <= 128 (the planner checks it).
+__host__ __device__ inline bool att_p_fits_tmem(int M, int tc_cap) { return ((tc_cap + 15) / 16) * (M / 128) <= 32; }
+
+__device__ __forceinline__ uint32_t att_p_taddr(uint32_t tmem_base) {
+  const int warp = threadIdx.x >> 5;
+  return tmem_base + ((uint32_t)(32 * (warp & 3)) << 16) + (uint32_t)((warp >> 2) * 128);
+}
+
+template <int N>
+__device__ __forceinline__ void tmem_st_32x32b(uint32_t taddr, const uint32_t (&v)[N]) {
+  static_assert(N == 4 || N == 8 || N == 16, "4, 8 or 16 columns");
+  if constexpr (N == 4) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x4.b32 [%0], {%1, %2, %3, %4};\n"
+                 ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]) : "memory");
+  } else if constexpr (N == 8) {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};\n"
+                 ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
+                 : "memory");
+  } else {
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], "
+                 "{%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};\n"
+                 ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]),
+                 "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15])
+                 : "memory");
+  }
+}
+
+// load + wait: the destination registers are complete when this returns
+template <int N>
+__device__ __forceinline__ void tmem_ld_32x32b(uint32_t taddr, uint32_t (&v)[N]) {
+  static_assert(N == 4 || N == 8 || N == 16, "4, 8 or 16 columns");
+  if constexpr (N == 4) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x4.b32 {%0, %1, %2, %3}, [%4];\n"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]) : "r"(taddr));
+  } else if constexpr (N == 8) {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];\n"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7])
+                 : "r"(taddr));
+  } else {
+    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
+                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];\n"
+                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
+                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
+                 : "r"(taddr));
+  }
+  asm volatile("tcgen05.wait::ld.sync.aligned;\n" ::: "memory");
+}
+
+// One-time copy of P rows [t0, t0 + nt) of utterance column u into this thread's TMEM columns (layout above).
+// Tail rows >= nt are clamped to nt - 1 exactly as the L2 path of att_energies does.  All ATT_NT threads.
+template <int NTW>
+__device__ __forceinline__ void att_stage_p_tmem_t(const float* P, int U, int M, int u, int t0, int nt, uint32_t taddr) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int g = lane >> 2, tig = lane & 3;
+  const float* pbase = P + ((long long)t0 * U + u) * M + warp * NTW * 8 + 2 * tig;
+  const long long prow = (long long)U * M;
+  const int ntile = (nt + 15) / 16;
+  for (int tile = 0; tile < ntile; ++tile) {
+    const int r0 = min(tile * 16 + g, nt - 1), r1 = min(tile * 16 + g + 8, nt - 1);
+    uint32_t v[4 * NTW];
+#pragma unroll
+    for (int j = 0; j < NTW; ++j) {
+      const float2 x0 = __ldg(reinterpret_cast<const float2*>(pbase + r0 * prow + j * 8));
+      const float2 x1 = __ldg(reinterpret_cast<const float2*>(pbase + r1 * prow + j * 8));
+      v[j * 4 + 0] = __float_as_uint(x0.x); v[j * 4 + 1] = __float_as_uint(x0.y);
+      v[j * 4 + 2] = __float_as_uint(x1.x); v[j * 4 + 3] = __float_as_uint(x1.y);
+    }
+    tmem_st_32x32b<4 * NTW>(taddr + (uint32_t)(tile * 4 * NTW), v);
+  }
+  asm volatile("tcgen05.wait::st.sync.aligned;\n" ::: "memory");
+}
+
+__device__ __forceinline__ void att_stage_p_tmem(const float* P, int U, int M, int u, int t0, int nt, uint32_t taddr) {
+  if (M == 512) att_stage_p_tmem_t<4>(P, U, M, u, t0, nt, taddr);
+  else if (M == 256) att_stage_p_tmem_t<2>(P, U, M, u, t0, nt, taddr);
+  else att_stage_p_tmem_t<1>(P, U, M, u, t0, nt, taddr);
+}
+
 // NTW: 8-column tiles of the matcher dimension per warp (M = 128 * NTW).
-template <int NTW, bool COMPACT>
+// P_TMEM: P comes from tensor memory (a.p_taddr, staged once by att_stage_p_tmem) instead of L2.
+template <int NTW, bool COMPACT, bool P_TMEM = false>
 __device__ __forceinline__ void att_energies(const AttRowIO& a, const AttSmem& s, int nt, int t0, int tc_cap) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int g = lane >> 2, tig = lane & 3;
@@ -198,9 +289,19 @@ __device__ __forceinline__ void att_energies(const AttRowIO& a, const AttSmem& s
       dst[j][1] = __ldg(reinterpret_cast<const float2*>(pbase + r1 * prow + j * 8));
     }
   };
-  if (ntile > 0) load_p(pc, 0);
+  if (!P_TMEM && ntile > 0) load_p(pc, 0);
   for (int tile = 0; tile < ntile; ++tile) {
-    if (tile + 1 < ntile) load_p(pn, tile + 1);
+    if constexpr (P_TMEM) {
+      uint32_t r[4 * NTW];
+      tmem_ld_32x32b<4 * NTW>(a.p_taddr + (uint32_t)(tile * 4 * NTW), r);
+#pragma unroll
+      for (int j = 0; j < NTW; ++j) {
+        pc[j][0] = make_float2(__uint_as_float(r[j * 4 + 0]), __uint_as_float(r[j * 4 + 1]));
+        pc[j][1] = make_float2(__uint_as_float(r[j * 4 + 2]), __uint_as_float(r[j * 4 + 3]));
+      }
+    } else if (tile + 1 < ntile) {
+      load_p(pn, tile + 1);
+    }
     const int ta = tile * 16 + g, tb = ta + 8;
     uint32_t ah[4], al[4];
     ah[0] = s.sF[(size_t)ta * 16 + tig];     ah[1] = s.sF[(size_t)tb * 16 + tig];
@@ -231,8 +332,10 @@ __device__ __forceinline__ void att_energies(const AttRowIO& a, const AttSmem& s
       part[ta] = ea;       // this warp's private partial sums; rows >= nt land in the 16-row padding
       part[tb] = eb;
     }
+    if constexpr (!P_TMEM) {
 #pragma unroll
-    for (int j = 0; j < NTW; ++j) { pc[j][0] = pn[j][0]; pc[j][1] = pn[j][1]; }
+      for (int j = 0; j < NTW; ++j) { pc[j][0] = pn[j][0]; pc[j][1] = pn[j][1]; }
+    }
   }
 }
 
@@ -247,7 +350,8 @@ __device__ __forceinline__ float gmax_of(const float* xs, int cs) {
 // sentinel-initialised buffers (common.cuh, "the data is the flag"): they are read with polling
 // loads and the outputs other CTAs consume are written with gpu-scope stores.
 // `entry_wait_pending`: the caller issued barrier.cluster.arrive at kernel entry.
-template <bool COMPACT = false>
+// P_TMEM_OK: compile the energy loop that reads P from tensor memory (taken when a.p_tmem is set).
+template <bool COMPACT = false, bool P_TMEM_OK = false>
 __device__ __forceinline__ void attention_row(const AttRowIO& a, float* smem, int tc_cap, int rank, int cs,
                                               bool constants_staged, bool flow,
                                               bool entry_wait_pending) {
@@ -354,9 +458,15 @@ __device__ __forceinline__ void attention_row(const AttRowIO& a, float* smem, in
   ATT_STAMP(2);
 
   // ---- energies: e[t] = v . tanh(P[t] + q + F[t] . Wh) on the tensor cores -------------
-  if (M == 512) att_energies<4, COMPACT>(a, s, nt, t0, tc_cap);
-  else if (M == 256) att_energies<2, COMPACT>(a, s, nt, t0, tc_cap);
-  else att_energies<1, COMPACT>(a, s, nt, t0, tc_cap);
+  if (P_TMEM_OK && a.p_tmem) {
+    if (M == 512) att_energies<4, COMPACT, P_TMEM_OK>(a, s, nt, t0, tc_cap);
+    else if (M == 256) att_energies<2, COMPACT, P_TMEM_OK>(a, s, nt, t0, tc_cap);
+    else att_energies<1, COMPACT, P_TMEM_OK>(a, s, nt, t0, tc_cap);
+  } else {
+    if (M == 512) att_energies<4, COMPACT>(a, s, nt, t0, tc_cap);
+    else if (M == 256) att_energies<2, COMPACT>(a, s, nt, t0, tc_cap);
+    else att_energies<1, COMPACT>(a, s, nt, t0, tc_cap);
+  }
   __syncthreads();
   {
     // e[t] = the 16 warps' partial sums, added in a fixed order

@@ -8,7 +8,10 @@
 //     slices of each CTA stay in SHARED MEMORY across all steps (2.75 MB spread over the
 //     grid), as do the attention constants (conv filters, handler, energy vector).
 //   * phase A (attention) is row-parallel: a cluster of `cs` CTAs per decoder row streams the
-//     row's P and H slices once and merges (max, sum, partial context) through DSMEM.
+//     row's P and H slices once and merges (max, sum, partial context) through DSMEM.  When the
+//     window is the whole utterance on every step (expanding prior that never cuts) and the CTA's
+//     P fragments fit its 512 TMEM columns, P is staged into tensor memory once per launch and the
+//     energies read it from there instead of from L2 (a.p_in_tmem, attention_row.cuh).
 //   * phases B1..B3 (gates, candidate, next query) are 2-D tiled skinny products:
 //     16-row x nc-column tiles, K split over the 16 warps of the CTA, fused GRU epilogues.  A CTA's
 //     gate tile and candidate tile cover the same units of the same rows, so update gate,
@@ -225,6 +228,24 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dec_scan_kernel(DecScanArgs a) 
     return;
   }
 
+  // ---- tensor memory for the resident P slice (a.p_in_tmem) ---------------------------------
+  // All 512 columns: the kernel runs one CTA per SM (its shared memory admits no second CTA of this or
+  // any other kernel that allocates tensor memory), so the allocation never waits for another owner.
+  // From here on every path reaches the dealloc at the end of the kernel.
+  uint32_t tmem_base = 0;
+  if (!COMPACT && a.p_in_tmem) {
+    uint32_t* slot = reinterpret_cast<uint32_t*>(smem + att_smem_floats(M, E, a.K, a.n, a.tc_cap, cs, a.wh_rows) - 16);
+    if (warp == 0) {
+      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;\n"
+                   ::"r"((uint32_t)__cvta_generic_to_shared(slot)), "r"(512u) : "memory");
+      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;\n" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+    tmem_base = *slot;
+  }
+
   // ---- who synchronises with whom --------------------------------------------------------
   // island mode: the batch is cut into islands of <= 16 rows; an island's CTAs (its rows'
   // attention clusters) also own the island's dense tiles, so islands never wait for each other.
@@ -283,6 +304,12 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dec_scan_kernel(DecScanArgs a) 
     w3s[(size_t)k * ws3 + c] = (in3 && col < M) ? a.Ws[(long long)k * M + col] : 0.f;
   }
   att_stage_constants(att_carve(att, M, E, a.K, a.n, a.tc_cap, cs, a.wh_rows), a.v, a.Wh, a.filt, M, a.K, a.n, a.wh_rows);
+  // the window is [0, T') on every step (planner): this CTA's positions are the same on every step
+  const uint32_t p_taddr = att_p_taddr(tmem_base);
+  if (!COMPACT && a.p_in_tmem && cluster_id < R) {
+    const int tc = (a.Tp + cs - 1) / cs, t0 = min(a.Tp, rank * tc), nt = min(a.Tp, t0 + tc) - t0;
+    att_stage_p_tmem(a.P, R, M, cluster_id, t0, nt, p_taddr);
+  }
   __syncthreads();
 
   // query of the first step: q = s_0 . W_state
@@ -372,7 +399,9 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dec_scan_kernel(DecScanArgs a) 
       io.rowpos_out = (a.prior.type == LVSR_PRIOR_EXPANDING) ? nullptr : (rowpos_wr + row);
       io.rowpos_mode = a.prior.type;
       io.trace = (a.trace && bid == 0) ? a.trace + (size_t)2 * a.L * 9 + (size_t)i * 8 : nullptr;
-      attention_row<COMPACT>(io, att, a.tc_cap, rank, cs, true, true, false);
+      io.p_tmem = a.p_in_tmem;
+      io.p_taddr = p_taddr;
+      attention_row<COMPACT, !COMPACT>(io, att, a.tc_cap, rank, cs, true, true, false);
     }
     DS_STAMP(1);
     if (a.trace && rank == 0 && tid == 0 && cluster_id < R)
@@ -414,7 +443,12 @@ __global__ void __launch_bounds__(DS_THREADS, 1) dec_scan_kernel(DecScanArgs a) 
       DS_STAMP(8);
     }
   }
+  if (!COMPACT && a.p_in_tmem) asm volatile("tcgen05.fence::before_thread_sync;\n" ::: "memory");
   cluster.sync();   // no CTA exits while a peer may still address its shared memory
+  if (!COMPACT && a.p_in_tmem && warp == 0) {
+    asm volatile("tcgen05.fence::after_thread_sync;\n" ::: "memory");
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;\n" ::"r"(tmem_base), "r"(512u) : "memory");
+  }
 }
 
 int sm_count() { return device_sm_count(); }
@@ -462,8 +496,26 @@ size_t derive(DecScanArgs& a, int cs, int G, bool want_islands) {
   return 0;
 }
 
+// Does the attention window cover the whole utterance on every step?  Only the expanding prior can say so
+// before the launch (b0 = 0 and b1 = T' for every i < L).  The bounds keep a margin of one position to the
+// device's rounding: a window that only just reaches an end takes the L2 path, which is always correct.
+bool window_is_whole_utterance(const DecScanArgs& a) {
+  if (a.prior.type != LVSR_PRIOR_EXPANDING) return false;
+  for (int i = 0; i < a.L; ++i) {
+    const double bb = a.prior.initial_begin + (double)i * a.prior.min_speed;
+    const double ee = a.prior.initial_end + (double)i * a.prior.max_speed;
+    if (!(bb < 1.0 - 1e-6) || !(ee > (double)(a.Tp - 1) + 1e-6)) return false;   // false on NaN too
+  }
+  return true;
+}
+
+// plan of the last plan_and_launch (lvsr_dec_scan_plan); cs = 0: the persistent decoder did not run
+struct DecScanPlan { int cs, islands, p_in_tmem; };
+DecScanPlan g_last_plan = {0, 0, 0};
+
 int plan_and_launch(DecScanArgs& a, int* supported, cudaStream_t stream) {
   *supported = 0;
+  g_last_plan = {0, 0, 0};
   const int sms = sm_count();
   const int R = a.B, C = a.C, E = a.E, M = a.M;
   if (!kper_ok(E + C) || !kper_ok(C) || !(M == 128 || M == 256 || M == 512) || E % 4 != 0 || E / 4 > DS_THREADS) return 0;
@@ -518,6 +570,13 @@ int plan_and_launch(DecScanArgs& a, int* supported, cudaStream_t stream) {
     }
     if (R * cs > G) continue;        // not enough clusters for one per row: try a smaller cluster
     {
+      // P in tensor memory: each CTA re-reads the same P slice on every step when the window is the whole
+      // utterance; keep it on chip if its fragments fit.  LVSR_DEC_TMEM_P=0 forces the L2 path (A/B runs).
+      const char* tp = getenv("LVSR_DEC_TMEM_P");
+      const bool allow = !(tp && strcmp(tp, "0") == 0);
+      a.p_in_tmem = (allow && !compact && att_p_fits_tmem(M, a.tc_cap) && window_is_whole_utterance(a)) ? 1 : 0;
+    }
+    {
       // profilers slow the kernel down by orders of magnitude: let them raise the hang guard
       const char* sl = getenv("LVSR_FLOW_SPIN_LIMIT");
       const unsigned lim = sl ? (unsigned)strtoul(sl, nullptr, 10) : LVSR_SPIN_LIMIT;
@@ -532,6 +591,7 @@ int plan_and_launch(DecScanArgs& a, int* supported, cudaStream_t stream) {
     }
     g_launch_count++;
     *supported = 1;
+    g_last_plan = {cs, islands ? 1 : 0, a.p_in_tmem};
 #ifdef LVSR_DEC_DEBUG
     {
       LVSR_CUDA_OK(cudaStreamSynchronize(stream));
@@ -561,3 +621,10 @@ int dec_scan_try(DecScanArgs& a, int* supported, cudaStream_t stream) {
 }
 
 }  // namespace lvsr
+
+extern "C" int lvsr_dec_scan_plan(int* cs, int* islands, int* p_in_tmem) {
+  if (cs) *cs = lvsr::g_last_plan.cs;
+  if (islands) *islands = lvsr::g_last_plan.islands;
+  if (p_in_tmem) *p_in_tmem = lvsr::g_last_plan.p_in_tmem;
+  return 0;
+}

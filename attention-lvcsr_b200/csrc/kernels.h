@@ -192,6 +192,7 @@ struct DecScanArgs {
   int nisl, ncg;                       // nisl > 0: islands of <= 16 rows whose CTAs own their dense tiles
   int wh_rows;                         // handler rows in shared memory: 16 (fast) or K (compact, long utterances)
   int red_alias;                       // dense-tile scratch shares the attention reduction scratch (long utterances)
+  int p_in_tmem;                       // each CTA's P slice is staged once into tensor memory (whole-utterance window)
 };
 int dec_scan_try(DecScanArgs& a, int* supported, cudaStream_t stream);
 

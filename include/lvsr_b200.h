@@ -95,6 +95,11 @@ int lvsr_model_finalize(lvsr_model* m);
  * kernels by itself and counts it in *stepwise_fallbacks (may be NULL).  No reference counterpart:
  * Theano raises from inside the compiled function instead. */
 int lvsr_model_status(lvsr_model* m, int32_t* launch_status, int64_t* stepwise_fallbacks);
+/* Plan of the persistent decoder's last planning call in this process (any handle): cluster size
+ * (0 = the step-wise kernels ran instead), island mode, and whether each CTA kept its slice of the
+ * preprocessed context in tensor memory (whole-utterance windows only; LVSR_DEC_TMEM_P=0 turns it off).
+ * Any pointer may be NULL.  Host-only, does not synchronise. */
+int lvsr_dec_scan_plan(int* cs, int* islands, int* p_in_tmem);
 
 /* ---- encoder: BeamSearch.context_computer / Encoder.apply -------------------------
  * (libs/blocks/blocks/search.py:97-99; lvsr/bricks/__init__.py:71-78).
